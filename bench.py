@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """EfficientDet hot-path throughput on N B200s of one node (BASELINE.json metric and configs).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config d0|d4|d7]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config d0|d4|d7] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0) as .npy files: inputs, weights and
+the drop-connect stream are seeded, so two builds run with the same arguments can be compared output for output.
 
 --config d0 (default, BASELINE.json configs[1]/[2], the headline metric): EfficientDet-D0 512x512, bs=32 per GPU.
   A "step" = one pass of the hot path over one synthetic batch: backbone -> BiFPN -> head -> FocalLoss forward, then
@@ -121,6 +124,27 @@ def usable_cores():
 def synthetic(cfgd, B, seed):
     import effdet_oracle as O
     return O.synthetic_batch(B, size=cfgd['size'], G=G_ANN, num_classes=cfgd['K'], seed=seed)
+
+
+DUMP_BYTES = 60 << 20          # data of all dumped arrays together; with the .npy headers the dump stays under 64 MB
+
+
+def dump_outputs(outputs, path):
+    """Write each named tensor of `outputs` as <path>/<name>.npy: float32, or float64 for integer tensors (exact).
+    When they exceed DUMP_BYTES together, every tensor is cut to the same fraction of its elements, at sorted indices
+    drawn by a generator seeded with 0, so two runs or two builds with the same arguments store the same elements."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    outputs = {k: v.detach() for k, v in outputs.items() if v is not None}
+    total = sum(v.numel() * (4 if v.is_floating_point() else 8) for v in outputs.values())
+    frac = min(1.0, DUMP_BYTES / max(total, 1))
+    for name, t in outputs.items():
+        if frac < 1.0:
+            n = max(1, int(t.numel() * frac))
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(path, name + '.npy'), a.astype(np.float32 if t.is_floating_point() else np.float64))
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -287,6 +311,7 @@ def run_ours(args):
                                                             broadcast_buffers=os.environ.get('EFFDET_DDP_BCAST', '0') == '1')
         torch.cuda.current_stream(dev).wait_stream(side)
 
+    torch.manual_seed(0)               # drop-connect masks: the same random stream on every run with the same arguments
     images_h, ann_h = synthetic(cfgd, BS, seed=1000 + rank)
     images_h, ann_h = images_h.pin_memory(), ann_h.pin_memory()
     images_d, ann_d = images_h.to(dev), ann_h.to(dev)
@@ -299,7 +324,7 @@ def run_ours(args):
             cl, rl = (module or net)([x, a])
             loss = cl.mean() + rl.mean()
             loss.backward()
-            return loss
+            return loss.detach()
     else:
         def step(x, a, module=None):
             with torch.no_grad():
@@ -358,8 +383,17 @@ def run_ours(args):
     if rank == 0:                      # one nvidia-smi poller per job, on rank 0's GPU
         sampler.start()
     _native.reset_launch_count()
-    ms = timed(lambda: step(images_d, ann_d), args.steps)
+    ms = timed(lambda: last.__setitem__('out', step(images_d, ann_d)), args.steps)
     launches = graph_launches if graphed is not None else _native.launch_count() // max(args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed step receives from its last step, before any later step overwrites it: the loss
+        # and every parameter gradient (train), or the detections of image 0 (inference)
+        if train:
+            outs = {'loss': last['out']}
+            outs.update(('grad.' + k, p.grad) for k, p in model.named_parameters())
+        else:
+            outs = dict(zip(('scores', 'classes', 'boxes'), last['out']))
+        dump_outputs(outs, args.dump_outputs)
 
     # host-side issue time of one step (queue empty before, no sync after): how far the CPU runs ahead of the GPU
     torch.cuda.synchronize()
@@ -501,7 +535,11 @@ def main():
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg (profiling runs)')
     ap.add_argument('--no-graph', action='store_true', help='issue every launch from Python instead of replaying a CUDA graph')
     ap.add_argument('--full-breakdown', action='store_true', help='list every kernel class in kernel_breakdown')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps write what the last one computed '
+                    '(loss and parameter gradients, or detections) as DIR/<name>.npy, at most 64 MB in all')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -135,7 +135,9 @@ def run_forward_case(tag, cfg, mode, size, B, seed, threshold=None):
     print('%-28s ok: %d tensors pinned, %d detections' % (tag, len(store), det_ref[0].numel()))
 
 
-def run_train_case(tag, cfg, size, B, seed, empty_first):
+def run_train_case(tag, cfg, size, B, seed, empty_first, samples=True):
+    """samples=False leaves out the sampled large gradients (gsamp/), which only the D0 GPU test reads: the D4 file
+    stays under 1 MB with every full gradient and every norm kept"""
     sd = O.init_state_dict(cfg, seed=seed, mode='wellcond')
     ref = build_reference(cfg, sd, is_training=True)
     ref.eval()                 # no drop-connect; BN is frozen in either mode
@@ -169,7 +171,7 @@ def run_train_case(tag, cfg, size, B, seed, empty_first):
         norms.append(float(torch.linalg.vector_norm(g.double())))
         if g.numel() <= 4096 or k.endswith('w1') or k.endswith('w2'):
             store['grad/' + k] = g.numpy().copy()
-        else:
+        elif samples:
             v, idx = sample(g, 129)
             store['gsamp/' + k + '/s'] = v
             store['gsamp/' + k + '/i'] = idx
@@ -226,7 +228,7 @@ if __name__ == '__main__':
         ('d0_256_train_b2_empty', run_train_case, (d0s, 256, 2, 4, True)),
         ('d1_384_fwd_wellcond', run_forward_case, (d1, 'wellcond', 384, 1, 5)),
         ('d4_256_fwd_wellcond', run_forward_case, (d4, 'wellcond', 256, 1, 6, 0.05)),
-        ('d4_128_train_b2', run_train_case, (d4, 128, 2, 7, False)),
+        ('d4_128_train_b2', run_train_case, (d4, 128, 2, 7, False, False)),
         ('d7_256_fwd_wellcond', run_forward_case, (d7, 'wellcond', 256, 1, 8, 0.05)),
     ]
     for tag, fn, a in cases:

@@ -12,6 +12,16 @@ import effdet_oracle as O
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
 
+@pytest.fixture(autouse=True)
+def golden_threads():
+    """torch's CPU convolutions split their work by thread count and the bits depend on the split: run at the 8 threads
+    the goldens were captured with (make_golden.py), whatever the host's core count or an earlier test set"""
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)
+
+
 def _check(store, name, t):
     s, i = store[name + '/s'], store[name + '/i']
     assert tuple(store[name + '/shape']) == tuple(t.shape), name
